@@ -274,7 +274,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side", action="store_true", help="skip the side measurements (q_sweep, c5, l2, small files, digest set)")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.rows == 0:
         args.rows = 12_500_000 if (world == 8 and args.impl == "ours") else REF_ROWS
@@ -317,9 +321,10 @@ def main():
         return [float(-t[1].item()), float(t[0].item())]
 
     out = {}
-    W, K = max(args.warmup, 0), max(args.steps, 1)
+    W, K = max(args.warmup, 0), args.steps
     sampler = ClockSampler(local)
     side = {}          # work for after the GPU-timed regions (checker / CPU legs)
+    dumps = {}         # --dump-outputs: name -> array
 
     # ------------------------------------------------------------------ knn -------------------------
     if args.workload in ("both", "knn"):
@@ -386,6 +391,15 @@ def main():
         e1.record(S)
         barrier_sync()
         ms_total = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:       # the top-k the last timed step handed to its caller (merged over ranks at N > 1)
+            b = (K - 1) & 1
+            if dist:
+                last_r, last_s = fin_r[b].cpu().numpy(), fin_s[b].cpu().numpy()
+            else:
+                packed = part[b].cpu().numpy()
+                last_r, last_s = packed[:nq * k * 8].view(np.int64), packed[nq * k * 8:].view(np.float32)
+            dumps["knn_rowids"] = last_r.reshape(nq, k).astype(np.float64)
+            dumps["knn_scores"] = last_s.reshape(nq, k).astype(np.float32)
         if dist:
             gather_ms = [ev_c[i][0].elapsed_time(ev_c[i][1]) for i in range(K)]
             merge_ms = [ev_c[i][1].elapsed_time(ev_c[i][2]) for i in range(K)]
@@ -680,7 +694,7 @@ def main():
         buf = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
         Y.synth_bytes_device(12345 + rank, 0, nbytes, buf.data_ptr())
         cfg = Y.default_config()
-        Wi, Ki = min(max(W, 1), 3), min(K, 5)
+        Wi, Ki = min(max(W, 1), 3), K
         for _ in range(Wi):
             ch = Y.chunk_and_hash_device(buf.data_ptr(), nbytes, cfg)
         barrier_sync()
@@ -691,6 +705,12 @@ def main():
             tot.append(t["total_ms"]); sha.append(t["sha256_ms"]); scan.append(t["scan_ms"]); sel.append(t["select_ms"])
         barrier_sync()
         ms = max_over_ranks(float(np.mean(tot)))
+        if args.dump_outputs and rank == 0:       # the chunk table of the last timed step: its size and a fixed, seeded sample of rows
+            pick = np.sort(np.random.default_rng(0).choice(len(ch), size=min(len(ch), 1 << 16), replace=False))
+            dumps["ingest_chunk_count"] = np.array([len(ch)], dtype=np.float64)
+            dumps["ingest_offset"] = ch["offset"][pick].astype(np.float64)
+            dumps["ingest_size"] = ch["size"][pick].astype(np.float64)
+            dumps["ingest_digest_words"] = np.ascontiguousarray(ch["digest"][pick]).view(">u4").astype(np.float64)   # 8 big-endian words
         gbs = nbytes / (ms / 1e3) / 1e9 * world
         sha_gbs = nbytes / (float(np.mean(sha)) / 1e3) / 1e9
         scan_gbs = nbytes / (float(np.mean(scan)) / 1e3) / 1e9
@@ -864,6 +884,10 @@ def main():
                 if args.workload == "ingest":
                     out["cpu_baseline"] = out["ingest"]["cpu_baseline"]
 
+    if dumps:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         print(json.dumps(out), flush=True)
     if dist:

@@ -3,6 +3,8 @@ bruteForceSearchUnlocked / vec0_run_exact_query and the reference golden vectors
 import numpy as np
 import pytest
 
+from tests.refdata import expect
+
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-4   # the reference tests' own epsilon (sqlite-vec-cpp/tests/test_distances.cpp:16-18)
@@ -337,27 +339,31 @@ def test_pairwise_and_batch_operators_are_bit_identical_to_the_reference_build(Y
     """R5/R6/R7: distances::{l2,cosine}_distance<float> in the operation order of the reference build (AVX lanes, FMA contraction
     where the compiler applies it) -- compared bit for bit with the reference compiled in place, at dims that take every path."""
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs the reference compiled in place")
-    R = O.ref()
+
+    def ref_dist(fn, q, rows):
+        R = O.ref()
+        return [getattr(R, fn)(O._p(q, O.f32p), O._p(np.ascontiguousarray(r), O.f32p), len(q)) for r in rows]
     rng = np.random.default_rng(9)
     for d in (1, 5, 7, 8, 13, 16, 31, 32, 100, 384, 768, 1536):
-        for _ in range(6):
+        for t in range(6):
             a = rng.normal(size=d).astype(np.float32)
             b = rng.normal(size=d).astype(np.float32)
+            want_l2, want_cos = expect(f"knn.pairwise.{d}.{t}", lambda: np.array(
+                ref_dist("ref_l2_distance", a, [b]) + ref_dist("ref_cosine_distance", a, [b]), dtype=np.float32))
             rc, got = Y.vec_distance_l2(a, b)
-            assert rc == 0 and np.float32(got) == np.float32(R.ref_l2_distance(O._p(a, O.f32p), O._p(b, O.f32p), d)), ("l2", d)
+            assert rc == 0 and np.float32(got) == want_l2, ("l2", d)
             rc, got = Y.vec_distance_cosine(a, b)
-            assert rc == 0 and np.float32(got) == np.float32(R.ref_cosine_distance(O._p(a, O.f32p), O._p(b, O.f32p), d)), ("cos", d)
+            assert rc == 0 and np.float32(got) == want_cos, ("cos", d)
     for d, n in ((768, 4000), (100, 3000), (16, 500)):
         rows = rng.normal(size=(n, d)).astype(np.float32)
         q = rng.normal(size=d).astype(np.float32)
-        for metric, om, fn in ((Y.COSINE, O.METRIC_COSINE, R.ref_cosine_distance), (Y.L2, O.METRIC_L2, R.ref_l2_distance)):
+        for metric, om, fn in ((Y.COSINE, O.METRIC_COSINE, "ref_cosine_distance"), (Y.L2, O.METRIC_L2, "ref_l2_distance")):
             got = Y.batch_distance(q, rows, metric=metric, mode=Y.BATCH_ALL)
-            want = np.array([fn(O._p(q, O.f32p), O._p(np.ascontiguousarray(rows[i]), O.f32p), d) for i in range(n)], dtype=np.float32)
+            want = expect(f"knn.batch_all.{d}.{metric}", lambda: np.array(ref_dist(fn, q, rows), dtype=np.float32))
             assert np.array_equal(got, want), (metric, d)
             idx, dist = Y.batch_distance(q, rows, metric=metric, mode=Y.BATCH_TOP_K, k=10)
-            ri, rd = O.batch_top_k(q, rows, 10, metric=om, use_ref=True)
+            ri = expect(f"knn.batch_top_k.{d}.{metric}.idx", lambda: O.batch_top_k(q, rows, 10, metric=om, use_ref=True)[0])
+            rd = expect(f"knn.batch_top_k.{d}.{metric}.dist", lambda: O.batch_top_k(q, rows, 10, metric=om, use_ref=True)[1])
             assert np.array_equal(dist, rd) and (list(idx) == list(ri) or len(set(rd)) < 10)
     # L1 (the SQL scalar vec_distance_l1): both paths of distances/l1.hpp against a float64 evaluation
     for d in (3, 7, 8, 100):

@@ -4,6 +4,8 @@ simeonPqSearchUnlocked (src/vector/sqlite_vec_backend.cpp:3868-4056) around them
 import numpy as np
 import pytest
 
+from tests.refdata import digest, expect
+
 pytestmark = pytest.mark.gpu
 
 
@@ -15,7 +17,14 @@ def Y():
     return yams_b200
 
 
-def reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, query, k, rerank, threshold):
+def reference_pq_search(O, key, rows, rowids, tie_keys, codebooks, m, kc, query, k, rerank, threshold):
+    """simeonPqSearchUnlocked's answer -> (rowids, scores), as recorded from simeon's own PQ code (tests/refdata.py)."""
+    got = expect(key, lambda: np.array(_reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, query, k, rerank, threshold),
+                                       dtype=np.float64).reshape(2, -1))
+    return [int(r) for r in got[0]], [np.float32(x) for x in got[1]]
+
+
+def _reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, query, k, rerank, threshold):
     """simeonPqSearchUnlocked, line by line, over simeon's own PQ code (oracle/_ref)."""
     n, d = rows.shape
     normed, ok = O.normalize_like_reference(rows)
@@ -43,8 +52,6 @@ def reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, query, k, r
 @pytest.mark.parametrize("cfg", [(12_000, 768, 32, 256), (9_000, 384, 32, 256), (20_000, 128, 8, 64), (5_000, 96, 4, 16)])
 def test_pq_index_and_search_match_the_reference_engine(Y, oracle, cfg):
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon's pq.cpp compiled in place")
     n, d, m, kc = cfg
     rng = np.random.default_rng(n)
     rows = O.gen_rows_f32(42, 0, n, d) * rng.uniform(0.5, 3.0, size=(n, 1)).astype(np.float32)   # not unit length: the index normalises
@@ -54,7 +61,7 @@ def test_pq_index_and_search_match_the_reference_engine(Y, oracle, cfg):
     tie_keys = rng.integers(0, 1 << 62, size=n).astype(np.uint64)
     normed, ok = O.normalize_like_reference(rows)
     if (n, d) == (20_000, 128):
-        codebooks = O.pq_train_ref(d, m, kc, normed[:4096])                         # the reference's own Lloyd training
+        codebooks = expect(f"pq.train.{n}.{d}.{m}.{kc}", lambda: O.pq_train_ref(d, m, kc, normed[:4096]))   # the reference's own Lloyd training
     else:
         codebooks = (rng.normal(size=(m, kc, d // m)) / np.sqrt(d)).astype(np.float32).reshape(-1)
     c = Y.Corpus(d, Y.F32, Y.COSINE)
@@ -62,13 +69,15 @@ def test_pq_index_and_search_match_the_reference_engine(Y, oracle, cfg):
     pq = Y.PqIndex(c, m, kc, codebooks, tie_break_keys=tie_keys)
     codes, code_rowids = pq.codes()
     assert np.array_equal(code_rowids, rowids[ok]) and len(codes) == n - 1
-    assert np.array_equal(codes, O.pq_encode_ref(codebooks, d, m, kc, normed))      # every code byte equals simeon's encode
+    assert np.array_equal(digest(codes), expect(f"pq.codes.{n}.{d}.{m}.{kc}",       # every code byte equals simeon's encode
+                                                lambda: digest(O.pq_encode_ref(codebooks, d, m, kc, normed))))
     queries = O.gen_rows_f32(43, 0, 6, d) * np.float32(2.0)
     queries[2] = rows[n // 3] * np.float32(0.5)                                     # hits the duplicated row pair
     for k, rerank, thr in ((10, 2, 0.0), (5, 4, -1.0), (25, 1, 0.1)):
         rid, sc, cnt, flags = pq.search(queries, k, rerank_factor=rerank, threshold=thr)
         for qi in range(len(queries)):
-            wr, ws = reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, queries[qi], k, rerank, thr)
+            wr, ws = reference_pq_search(O, f"pq.search.{n}.{d}.{m}.{kc}.{k}.{rerank}.{thr}.{qi}", rows, rowids, tie_keys, codebooks, m, kc,
+                                         queries[qi], k, rerank, thr)
             assert cnt[qi] == len(wr), (qi, k)
             assert list(rid[qi, :len(wr)]) == wr, (qi, k)
             assert np.array_equal(sc[qi, :len(wr)], np.array(ws, dtype=np.float32)), (qi, k)
@@ -88,8 +97,6 @@ def test_pq_over_an_fp16_corpus_and_row_order_ties(Y, oracle):
     """fp16 corpus (the C2 layout): the index is built from the stored (fp16) values; without tie keys equal approximate
     scores are ordered by row."""
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon's pq.cpp compiled in place")
     n, d, m, kc = 12_000, 256, 16, 256
     rng = np.random.default_rng(3)
     rows16 = O.f16_from_float(O.gen_rows_f32(42, 0, n, d)).reshape(n, d)
@@ -105,17 +112,17 @@ def test_pq_over_an_fp16_corpus_and_row_order_ties(Y, oracle):
     rid, sc, cnt, flags = pq.search(queries, 10, rerank_factor=2, threshold=-1.0)
     tie = np.arange(n, dtype=np.uint64)
     for qi in range(4):
-        wr, ws = reference_pq_search(O, rows, np.arange(n), tie, codebooks, m, kc, queries[qi], 10, 2, -1.0)
+        wr, ws = reference_pq_search(O, f"pq.fp16.{qi}", rows, np.arange(n), tie, codebooks, m, kc, queries[qi], 10, 2, -1.0)
         assert list(rid[qi, :len(wr)]) == wr and np.array_equal(sc[qi, :len(wr)], np.array(ws, dtype=np.float32))
     assert list(rid[1, :2]) == [50, 100] and flags[1] & Y.FLAG_TIE_AT_K == 0
     pq.close()
     c.close()
 
 
-def _check_against_reference(O, pq, rows, rowids, tie_keys, codebooks, m, kc, queries, k, rerank, thr):
+def _check_against_reference(O, key, pq, rows, rowids, tie_keys, codebooks, m, kc, queries, k, rerank, thr):
     rid, sc, cnt, flags = pq.search(queries, k, rerank_factor=rerank, threshold=thr)
     for qi in range(len(queries)):
-        wr, ws = reference_pq_search(O, rows, rowids, tie_keys, codebooks, m, kc, queries[qi], k, rerank, thr)
+        wr, ws = reference_pq_search(O, f"{key}.{k}.{rerank}.{thr}.{qi}", rows, rowids, tie_keys, codebooks, m, kc, queries[qi], k, rerank, thr)
         assert cnt[qi] == len(wr), (qi, k)
         assert list(rid[qi, :len(wr)]) == wr, (qi, k)
         assert np.array_equal(sc[qi, :len(wr)], np.array(ws, dtype=np.float32)), (qi, k)
@@ -125,8 +132,6 @@ def test_pq_filtered_scan_large_index(Y, oracle):
     """>= 64 tiles: the sampled-threshold (filtered) ADC pass replaces the per-tile sorting network; 1, 2 and 5 queries walk the
     1-, 2- and 4-table CTA variants.  Small k (16 centroids) makes equal approximate scores common: tie keys decide."""
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon's pq.cpp compiled in place")
     n, d, m, kc = 300_000, 64, 8, 16
     rng = np.random.default_rng(11)
     rows = O.gen_rows_f32(42, 0, n, d)
@@ -141,7 +146,7 @@ def test_pq_filtered_scan_large_index(Y, oracle):
     queries[1] = rows[2000]
     for nq in (1, 2, 5):
         for k, rerank, thr in ((10, 2, -1.0), (40, 3, 0.0)):
-            _check_against_reference(O, pq, rows, rowids, tie_keys, codebooks, m, kc, queries[:nq], k, rerank, thr)
+            _check_against_reference(O, f"pq.filtered.{nq}", pq, rows, rowids, tie_keys, codebooks, m, kc, queries[:nq], k, rerank, thr)
     pq.close()
     c.close()
 
@@ -150,8 +155,6 @@ def test_pq_filtered_scan_overflow_falls_back(Y, oracle):
     """The sampled tiles (every 4th of 74) hold only rows pointing away from the query, every other tile rows pointing at it:
     the sample's threshold admits ~237 k rows into a 32 k list; the engine must notice and redo the selection unfiltered."""
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon's pq.cpp compiled in place")
     n, d, m, kc = 300_000, 64, 8, 16
     rng = np.random.default_rng(12)
     query = O.gen_rows_f32(43, 0, 1, d)
@@ -165,6 +168,6 @@ def test_pq_filtered_scan_overflow_falls_back(Y, oracle):
     c = Y.Corpus(d, Y.F32, Y.COSINE)
     c.append(rows, rowids=rowids)
     pq = Y.PqIndex(c, m, kc, codebooks, tie_break_keys=tie_keys)
-    _check_against_reference(O, pq, rows, rowids, tie_keys, codebooks, m, kc, query, 10, 2, -1.0)
+    _check_against_reference(O, "pq.overflow", pq, rows, rowids, tie_keys, codebooks, m, kc, query, 10, 2, -1.0)
     pq.close()
     c.close()

@@ -3,6 +3,8 @@
 import numpy as np
 import pytest
 
+from tests.refdata import digest, expect
+
 pytestmark = pytest.mark.gpu
 
 
@@ -39,15 +41,14 @@ def corpus_of_texts(rng, n):
 ])
 def test_simeon_encoder_is_bit_identical(Y, oracle, cfg):
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon compiled in place")
     rng = np.random.default_rng(len(cfg) + 1)
     texts = corpus_of_texts(rng, 300)
     enc = Y.SimeonEncoder(**cfg)
     got = enc.encode(texts)
-    want = O.simeon_encode_ref(texts, **cfg)
-    assert got.shape == want.shape
-    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
+    key = "simeon.v1." + ".".join(f"{k}={v}" for k, v in sorted(cfg.items()))
+    shape = expect(key + ".shape", lambda: O.simeon_encode_ref(texts, **cfg).shape)
+    assert got.shape == tuple(shape)
+    assert np.array_equal(digest(got.view(np.uint32)), expect(key + ".digest", lambda: digest(O.simeon_encode_ref(texts, **cfg).view(np.uint32))))
     if cfg.get("l2_normalize", 1):
         norms = np.linalg.norm(got.astype(np.float64), axis=1)
         assert np.all((np.abs(norms - 1) < 1e-5) | (norms == 0))    # texts shorter than ngram_min embed to zero
@@ -84,19 +85,20 @@ def test_simeon_yams_default_profile_is_bit_identical(Y, oracle, cfg):
     """The encoder an unconfigured YAMS builds (simeon_embedding_backend.cpp:18-47,118-135): byte n-grams + word tokens, count
     sketch, FWHT projection, L2 -- against simeon's own Encoder with ngram_mode / projection set the same way."""
     O = oracle
-    if not O.ref_available():
-        pytest.skip("needs simeon compiled in place")
     rng = np.random.default_rng(123)
     texts = corpus_of_texts(rng, 300) + [b"_", b"a_b c-d e.f 0x1F", b"word" * 3000, b"  leading and trailing  ", "Größe_42 naïve".encode()]
     enc = Y.SimeonEncoder(**cfg)
     got = enc.encode(texts)
     c = enc.cfg
-    want = O.simeon_encode_modes_ref(texts, ngram_mode="CharAndWord" if c.flags & Y.SIMEON_WORD_TOKENS else "CharOnly",
-                                     projection="Fwht" if c.flags & Y.SIMEON_PROJECTION_FWHT else "AchlioptasSparse",
-                                     ngram_min=c.ngram_min, ngram_max=c.ngram_max, sketch_dim=c.sketch_dim, output_dim=c.output_dim,
-                                     hash_seed=c.hash_seed, projection_seed=c.projection_seed, l2_normalize=c.l2_normalize)
-    assert got.shape == want.shape
-    assert np.array_equal(got.view(np.uint32), want.view(np.uint32))
+
+    def want():
+        return O.simeon_encode_modes_ref(texts, ngram_mode="CharAndWord" if c.flags & Y.SIMEON_WORD_TOKENS else "CharOnly",
+                                         projection="Fwht" if c.flags & Y.SIMEON_PROJECTION_FWHT else "AchlioptasSparse",
+                                         ngram_min=c.ngram_min, ngram_max=c.ngram_max, sketch_dim=c.sketch_dim, output_dim=c.output_dim,
+                                         hash_seed=c.hash_seed, projection_seed=c.projection_seed, l2_normalize=c.l2_normalize)
+    key = "simeon.modes." + ".".join(f"{k}={v}" for k, v in sorted(cfg.items()))
+    assert got.shape == tuple(expect(key + ".shape", lambda: want().shape))
+    assert np.array_equal(digest(got.view(np.uint32)), expect(key + ".digest", lambda: digest(want().view(np.uint32))))
     assert np.array_equal(enc.encode([texts[7]])[0], got[7])
     enc.close()
     # the constraint of the reference constructor (projection.cpp:167-170)
