@@ -94,6 +94,11 @@ def lib():
         L.yo_cosine_distance_f32.argtypes = [f32p, f32p, C.c_size_t]
         L.yo_l2_distance_f32.restype = C.c_float
         L.yo_l2_distance_f32.argtypes = [f32p, f32p, C.c_size_t]
+        L.yo_l2_distance_build_f32.restype = C.c_float
+        L.yo_l2_distance_build_f32.argtypes = [f32p, f32p, C.c_size_t]
+        L.yo_exact_scan_l2_batch.restype = None
+        L.yo_exact_scan_l2_batch.argtypes = [C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, f32p, C.c_size_t, C.c_size_t,
+                                             i64p, f32p, u32p]
         L.yo_cosine_similarity_f64.restype = C.c_double
         L.yo_cosine_similarity_f64.argtypes = [f32p, f32p, C.c_size_t]
         L.yo_vec_distance_l2.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, f32p]
@@ -434,6 +439,33 @@ def exact_scan_cosine_batch(rows: np.ndarray, queries: np.ndarray, k: int, thres
                                           nq, k, threshold, _p(out_r, i64p), _p(out_s, f32p),
                                           _p(cnt, u32p))
     return rc, out_r, out_s, cnt
+
+
+def l2_distance_build(a: np.ndarray, b: np.ndarray) -> float:
+    """l2_distance<float> in the reference build's operation order (AVX lanes when d % 16 == 0, else the scalar loop)."""
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    b = np.ascontiguousarray(b, dtype=np.float32)
+    assert a.shape == b.shape and a.ndim == 1
+    return lib().yo_l2_distance_build_f32(_p(a, f32p), _p(b, f32p), a.size)
+
+
+def exact_scan_l2_batch(rows: np.ndarray, queries: np.ndarray, k: int):
+    """Exact L2 top-k of every query, distances in the reference build's order -> (rowids i64[Q,k], dist f32[Q,k],
+    counts u32[Q]); ties by row index, padding rowid -1 / +inf.  rows fp32 [n,d] or uint16 (fp16 bits) [n,d]."""
+    rows = np.ascontiguousarray(rows)
+    dtype = DTYPE_F16 if rows.dtype == np.uint16 else DTYPE_F32
+    if dtype == DTYPE_F32:
+        rows = rows.astype(np.float32, copy=False)
+    n, d = rows.shape
+    q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, d)
+    nq = q.shape[0]
+    out_r = np.full((nq, k), -1, dtype=np.int64)
+    out_d = np.full((nq, k), np.inf, dtype=np.float32)
+    cnt = np.zeros(nq, dtype=np.uint32)
+    if nq and k:
+        lib().yo_exact_scan_l2_batch(rows.ctypes.data_as(C.c_void_p), dtype, n, d, _p(q, f32p), nq, k, _p(out_r, i64p),
+                                     _p(out_d, f32p), _p(cnt, u32p))
+    return out_r, out_d, cnt
 
 
 def vec0_exact(rows: np.ndarray, query: np.ndarray, k: int = 0, rowids=None, rowid_range=None):

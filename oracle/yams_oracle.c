@@ -421,6 +421,26 @@ float yo_l2_distance_f32(const float* a, const float* b, size_t d) {
     return sqrtf(sum);
 }
 
+float yo_l2_distance_build_f32(const float* a, const float* b, size_t d) {
+    /* The build compiles distances/simd/avx.hpp (SQLITE_VEC_ENABLE_AVX, no FMA macro): one 8-float accumulator, so lane l
+     * sums the elements c + l, c = 0, 8, 16, ...; each (a - b)^2 is a rounded product added with its own rounding; the
+     * 8 lanes are then added left to right.  The vector path runs for d >= 16 && d % 16 == 0 only. */
+    if (d >= 16 && d % 16 == 0) {
+        float p[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        for (size_t c = 0; c < d; c += 8) {
+            for (int l = 0; l < 8; ++l) {
+                float diff = a[c + l] - b[c + l];
+                float sq = diff * diff;
+                p[l] = p[l] + sq;
+            }
+        }
+        float sum = p[0];
+        for (int l = 1; l < 8; ++l) sum = sum + p[l];
+        return sqrtf(sum);
+    }
+    return yo_l2_distance_f32(a, b, d);
+}
+
 double yo_cosine_similarity_f64(const float* a, const float* b, size_t d) {
     /* src/vector/vector_database.cpp:1786-1810 */
     double dp = 0.0, na = 0.0, nb = 0.0;
@@ -607,6 +627,47 @@ int yo_vec0_exact(const float* rows, size_t n, size_t d, const int64_t* rowids, 
     *out_count = cnt;
     free(res);
     return 0;
+}
+
+void yo_exact_scan_l2_batch(const void* rows, int dtype, size_t n, size_t d, const float* queries, size_t nq,
+                            size_t k, int64_t* out_rowids, float* out_dist, uint32_t* out_counts) {
+    static float f16_table[65536];
+    static int f16_table_ready = 0;
+    if (dtype == YO_DTYPE_F16 && !f16_table_ready) {
+        for (uint32_t h = 0; h < 65536; ++h) f16_table[h] = yo_f16_to_float((uint16_t)h);
+        f16_table_ready = 1;
+    }
+    const float* r32 = (const float*)rows;
+    const uint16_t* r16 = (const uint16_t*)rows;
+    long q;
+#pragma omp parallel for schedule(dynamic, 1)
+    for (q = 0; q < (long)nq; ++q) {
+        const float* qv = queries + (size_t)q * d;
+        distrow* res = (distrow*)malloc((n ? n : 1) * sizeof(distrow));
+        float* row = (float*)malloc((d ? d : 1) * sizeof(float));
+        size_t cnt = 0;
+        for (size_t r = 0; r < n; ++r) {
+            const float* rv = r32 + r * d;
+            if (dtype == YO_DTYPE_F16) {
+                for (size_t c = 0; c < d; ++c) row[c] = f16_table[r16[r * d + c]];
+                rv = row;
+            }
+            float dist = yo_l2_distance_build_f32(qv, rv, d);
+            if (dist != dist) continue;
+            res[cnt].dist = dist;
+            res[cnt].rowid = (int64_t)r;
+            ++cnt;
+        }
+        qsort(res, cnt, sizeof(distrow), cmp_dist);
+        size_t m = cnt < k ? cnt : k;
+        for (size_t i = 0; i < k; ++i) {
+            out_rowids[(size_t)q * k + i] = i < m ? res[i].rowid : -1;
+            out_dist[(size_t)q * k + i] = i < m ? res[i].dist : INFINITY;
+        }
+        out_counts[q] = (uint32_t)m;
+        free(row);
+        free(res);
+    }
 }
 
 size_t yo_batch_top_k(const float* query, const float* rows, size_t n, size_t d, int metric,

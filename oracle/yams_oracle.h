@@ -90,6 +90,10 @@ float yo_f16_to_float(uint16_t h);
 /* ---- distances (sqlite-vec-cpp distances/{cosine,l2}.hpp scalar paths) -------------------- */
 float yo_cosine_distance_f32(const float* a, const float* b, size_t d); /* cosine.hpp:48-69  */
 float yo_l2_distance_f32(const float* a, const float* b, size_t d);     /* l2.hpp:108-118    */
+/* l2_distance<float> in the operation order of the reference BUILD (sqlite-vec-cpp compiled with AVX, see
+ * yams_b200/csrc/ref_order.cuh): d >= 16 && d % 16 == 0 -> eight lane-strided float partial sums (multiply and add
+ * rounded separately), lanes summed left to right, sqrtf; otherwise the scalar loop of yo_l2_distance_f32. */
+float yo_l2_distance_build_f32(const float* a, const float* b, size_t d);
 /* vector_database.cpp:1786-1810 */
 double yo_cosine_similarity_f64(const float* a, const float* b, size_t d);
 /* sqlite_vec_c_api.cpp:57-105: returns 0 ok / 1 error, sizes in BYTES */
@@ -126,6 +130,13 @@ int yo_exact_scan_cosine_batch(const void* rows, int dtype, size_t n, size_t d,
 int yo_vec0_exact(const float* rows, size_t n, size_t d, const int64_t* rowids, const float* query,
                   size_t k, int use_range, int64_t rowid_lo, int64_t rowid_hi, int64_t* out_rowids,
                   float* out_dist, size_t* out_count);
+
+/* Exact L2 top-k of Q queries (OpenMP over queries) with yo_l2_distance_build_f32(query, row): the library's L2 search
+ * contract.  rows: n x d, fp32 or fp16 bit patterns (upcast exactly).  Order: distance asc, ties by row index asc; rows
+ * whose distance is NaN are left out.  out arrays are Q x k: count = min(k, rows kept), the rest padded with rowid -1
+ * and distance +inf. */
+void yo_exact_scan_l2_batch(const void* rows, int dtype, size_t n, size_t d, const float* queries, size_t nq,
+                            size_t k, int64_t* out_rowids, float* out_dist, uint32_t* out_counts);
 
 /* distances/batch.hpp:74-92 batch_top_k: indices of the k smallest distances (ties: index asc).
  * metric: YO_METRIC_COSINE uses cosine *distance*, YO_METRIC_L2 uses l2_distance. */

@@ -170,19 +170,18 @@ def test_vec0_exact_and_l2_surface(Y, oracle):
     big = O.gen_rows_f32(3, 0, 5000, 48)
     big[77] = big[5]
     q = O.gen_rows_f32(4, 0, 1, 48)[0]
+    # both against the exact L2 order of the reference build's own float distances (AVX lanes for d = 48): equal ids and
+    # bit-equal distances
     for k in (0, 25):
-        wr, wd = O.vec0_exact(big, q, k=k)
+        wr, wd, wc = O.exact_scan_l2_batch(big, q[None, :], k or len(big))
         rid, dist = Y.vec0_exact(q, big, k=k)
-        assert np.allclose(dist, wd, atol=TOL)
-        order_ok = list(rid) == list(wr)
-        if not order_ok:   # float summation order may swap near-equal neighbours: distances must agree
-            assert np.allclose(np.sort(dist), np.sort(wd), atol=TOL)
+        assert len(rid) == wc[0] and np.array_equal(rid, wr[0]) and np.array_equal(dist.view(np.uint32), wd[0].view(np.uint32))
     # corpus with the L2 metric (top-k ascending by distance)
     c = Y.Corpus(48, Y.F32, Y.L2)
     c.append(big)
     rid, sc, cnt, _ = c.search(q[None, :], 10)
-    wr, wd = O.vec0_exact(big, q, k=10)
-    assert cnt[0] == 10 and np.allclose(sc[0], wd, atol=TOL)
+    wr, wd, wc = O.exact_scan_l2_batch(big, q[None, :], 10)
+    assert np.array_equal(cnt, wc) and np.array_equal(rid, wr) and np.array_equal(sc.view(np.uint32), wd.view(np.uint32))
     c.close()
     # test_batch_distance.cpp:19-104 KATs through the same surface
     rows = np.array([[1, 2, 3], [2, 3, 4], [0, 0, 0], [4, 5, 6]], dtype=np.float32)

@@ -791,7 +791,8 @@ __global__ void rescore_kernel(const void* __restrict__ rows, int dtype, uint32_
 // a true score <= bound + eps.  The emitted top-k is provably the reference's top-k iff no such row can reach the k-th exact
 // score (or, with fewer than k valid survivors, the caller's threshold):
 //   cosine:  bound + eps <  (valid >= k ? sim_k : threshold)
-//   L2    :  |q|^2 - bound - eps > dist_k^2          (s~ = 2 q.r - |r|^2, so d^2 = |q|^2 - s)
+//   L2    :  (|q|^2 - bound - eps) (1 - g) > dist_k^2   (s~ = 2 q.r - |r|^2, so d^2 = |q|^2 - s; g: l2_rounding_slack)
+// Only bound == -inf (no row was left out) skips the test; a NaN bound or eps (stage-1 scores that overflowed) fails it.
 // Otherwise the query is queued for the exhaustive levels (status->bad / bad2) and flagged.
 struct CertArgs {
     const float* bound;       // per CTA
@@ -802,7 +803,21 @@ struct CertArgs {
     ScanStatus* status;       // nullable: no certificate (results already exhaustive)
     int level;                // 0: failures go to bad[], 1: to bad2[]
     uint32_t nq_total;        // capacity of each list
+    uint32_t dim;             // L2: rounding of |q|^2 in double
+    double l2_slack;          // L2: relative rounding error of the reference's float distance^2 (l2_rounding_slack)
 };
+
+// The reference's float L2 distance (ref_order.cuh) is dist~ = sqrtf(S~), S~ a float sum of the terms fl(fl(a - b)^2).
+// With u = 2^-24 and D the exact distance of the stored values: every term carries three roundings (the difference, counted
+// twice once squared, and the product), each term passes at most m rounded additions (scalar loop: m = d; AVX lanes: d/8
+// per lane plus 7 across the lanes, m = d/8 + 8 covers both), sqrtf rounds once more, counted twice in dist~^2.  So
+//   dist~^2 >= D^2 (1 - u)^(m + 5) >= D^2 (1 - (m + 5) u).
+// A row with D^2 >= L cannot reach dist_k (strictly) when L (1 - (m + 5) u) > dist_k^2.  For the scalar loop at d = 3000
+// g = 1.8e-4: the former flat 1e-4 was too small beyond d ~ 1650.
+static double l2_rounding_slack(uint32_t d) {
+    const double m = (d >= 16 && d % 16 == 0) ? d / 8.0 + 8.0 : (double)d;
+    return (m + 5.0) * 0x1p-24;
+}
 
 // one CTA per query: order survivors by (sim desc, row asc), emit k, certify.  CTA b serves query qmap[b] (or b).
 __global__ void __launch_bounds__(SEL_THREADS) final_kernel(const Exact* __restrict__ ex, const uint32_t* __restrict__ ex_n,
@@ -866,16 +881,17 @@ __global__ void __launch_bounds__(SEL_THREADS) final_kernel(const Exact* __restr
         if (cert.status && k > 0) {
             const float bd = cert.bound[b];
             bool certified = true;
-            if (bd > -INFINITY) {
+            if (bd != -INFINITY) {   // NaN included: the comparisons below are then false
                 const float e = cert.eps[q];
                 if (cert.metric == YAMS_B200_L2) {
                     certified = false;
                     if (valid >= k) {
                         const float dk = -fkey_inv((uint32_t)(buf[k - 1] >> 32));
                         const double qq = cert.qnorm[q] * cert.qnorm[q];
-                        // distances are floats of a float sum: allow their own rounding (d * 2^-24 relative, generously)
-                        const double dk2 = (double)dk * (double)dk * 1.0001 + 1e-30;
-                        certified = qq - (double)bd - (double)e > dk2;
+                        // lower bound of D^2 of every row not re-scored, less the double rounding of |q|^2 and of the difference
+                        const double lo = qq - (double)bd - (double)e;
+                        const double rnd = (double)(cert.dim + 4) * 0x1p-52 * (qq + fabs((double)bd) + (double)e);
+                        certified = (lo - rnd) * (1.0 - cert.l2_slack) > (double)dk * (double)dk;
                     }
                 } else {
                     const float lvl = valid >= k ? fkey_inv((uint32_t)(buf[k - 1] >> 32)) : cert.threshold;
@@ -1498,6 +1514,7 @@ static yams_status_t scan_enqueue(Corpus* c, const ScanPlan& p, int64_t* d_out_r
     CertArgs cert{};
     cert.bound = d_bound; cert.eps = c->eps.as<float>(); cert.qnorm = d_qnorm; cert.threshold = p.threshold;
     cert.metric = c->metric; cert.status = status_of(c); cert.level = 0; cert.nq_total = nq;
+    cert.dim = c->dim; cert.l2_slack = l2_rounding_slack(c->dim);
     final_kernel<<<nq, SEL_THREADS, 0, st>>>(d_ex, nullptr, Kp, k, c->rowids.as<int64_t>(), l2 ? 1 : 0, d_out_rowids, d_out_scores,
                                              d_out_counts, d_out_flags, l2 ? INFINITY : -INFINITY, nullptr, cert);
     YB_CUDA(cudaGetLastError());
@@ -1606,6 +1623,7 @@ static yams_status_t resolve_uncertain(Corpus* c, const ScanPlan& p, const uint3
         CertArgs cert{};
         cert.bound = d_bound1; cert.eps = c->eps2.as<float>(); cert.qnorm = d_qnorm; cert.threshold = p.threshold;
         cert.metric = c->metric; cert.status = status_of(c); cert.level = 1; cert.nq_total = p.nq;
+        cert.dim = c->dim; cert.l2_slack = l2_rounding_slack(c->dim);
         final_kernel<<<g, SEL_THREADS, 0, st>>>(d_ex1, d_sel1_n, K1, k, c->rowids.as<int64_t>(), l2 ? 1 : 0, d_out_rowids, d_out_scores,
                                                 d_out_counts, d_out_flags, l2 ? INFINITY : -INFINITY, d_qmap, cert);
         YB_CUDA(cudaGetLastError());
